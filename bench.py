@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            our CUDA path through the C-ABI (libbark_b200.so)
   python bench.py --impl reference --gpus N --steps K ...  the reference's own CPU path (oracle/_ref) on the host cores
+  --dump-outputs DIR                                         also write what the last timed step returned as DIR/<name>.npy
 
 Workload (BASELINE.json configs[1]): bark-small dimensions, f16 GPT + f16 codec, batch 1 per GPU, full
 semantic -> coarse -> fine -> EnCodec, synthetic seeded weights (no checkpoint is reachable offline), prompt
@@ -46,8 +47,12 @@ def metric_name(cfg):
     return f"audio sec/sec (inverse RTF), {BENCH_CONFIGS[cfg]['label']}, batch 1 per GPU, semantic->coarse->fine->encodec"
 PROMPT = "hello world"
 N_STEPS_TEXT = 138
+# the C oracle's bounded sample: 6 semantic steps -> 9 frames; 4 steps would give 6 frames, no more than the reflect padding of
+# the codec's first convolution (kernel 7), which the reference (ggml_pad_reflect_1d) and the oracle both reject
+PORT_STEPS = 6
 SAMPLE_RATE = 24000
-FIXTURE_DIR = os.environ.get("BARK_B200_FIXTURES", "/tmp/bark_b200_fixtures")
+# generated weight files, cached between runs; per user, since another user's directory of the same name is not writable
+FIXTURE_DIR = os.environ.get("BARK_B200_FIXTURES") or os.path.join(tempfile.gettempdir(), f"bark_b200_fixtures_{os.getuid()}")
 
 
 def peaks():
@@ -241,6 +246,7 @@ def run_ours(args):
     launches = pkg.kernel_launches() - launches0
     h2d, d2h = pkg.io_counters()
     n_audio = audio.size
+    last_outputs = dict(audio=audio, semantic_tokens=b.tokens(0), coarse_tokens=b.tokens(1), fine_tokens=b.tokens(2))
     s, pm = b.stats()
     n_samples = [pm[0][2], pm[1][2], pm[2][2]]        # cumulative since load (reference semantics, bark.cpp:1698)
     n_calls = args.warmup + args.steps
@@ -328,6 +334,8 @@ def run_ours(args):
     if dist:
         dist.destroy_process_group()
     emit(result)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_outputs)
     if not ok:
         sys.stderr.write("bench.py: PARITY FAILURE against the CPU reference on the benchmarked clip\n")
         sys.exit(3)
@@ -470,6 +478,8 @@ def run_fine_only(args):
                      "avg_launch_us": round(tv["ms"] * 1e3 / max(tv["launches"], 1), 2), "traffic": None, "peak_source": P["source"]},
         "kernels": {k: dict(launches=v["launches"], ms=round(v["ms"], 3)) for k, v in ranked[:8]},
     })
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(fine_tokens=tokens))
     if not ok:
         sys.stderr.write("bench.py: sharded fine tokens differ from the unsharded run\n")
         sys.exit(3)
@@ -530,10 +540,10 @@ def cpu_baseline(path, budget_s=30.0, steps=1, want_outputs=False):
                 "build": r.build_info(), "seconds": round(dt, 3)}
         return (base, g) if want_outputs else base
     orc.build_oracle()
-    o = orc.Oracle(path, seed=0, n_steps=4)
+    o = orc.Oracle(path, seed=0, n_steps=PORT_STEPS)
     t0 = time.perf_counter(); g = o.generate(PROMPT); dt = time.perf_counter() - t0
     base = {"value": round(g["audio"].size / SAMPLE_RATE / dt, 5), "unit": UNIT, "cores": cores, "kind": "port",
-            "sample": f"C oracle (OpenMP), bounded sample n_steps_text_encoder=4 -> {g['audio'].size / SAMPLE_RATE:.2f} s clip in {dt:.2f} s" + REF_2GIB_NOTE * (os.path.getsize(path) >= 2 ** 31),
+            "sample": f"C oracle (OpenMP), bounded sample n_steps_text_encoder={PORT_STEPS} -> {g['audio'].size / SAMPLE_RATE:.2f} s clip in {dt:.2f} s" + REF_2GIB_NOTE * (os.path.getsize(path) >= 2 ** 31),
             "seconds": round(dt, 3)}
     return (base, None) if want_outputs else base
 
@@ -564,7 +574,7 @@ def run_reference(args):
                   f"last step: semantic {st[2] / 1e3:.0f} ms, coarse {st[3] / 1e3:.0f} ms, fine {st[4] / 1e3:.0f} ms")
         build = r.build_info()
     else:
-        cores, n = os.cpu_count() or 1, 4
+        cores, n = os.cpu_count() or 1, PORT_STEPS
         orc.build_oracle()
         o = orc.Oracle(path, seed=0, n_steps=n)
         for i in range(args.warmup + args.steps):
@@ -583,6 +593,17 @@ def run_reference(args):
         "config": {"workload": f"{spec['label']}, batch=1, n_steps_text_encoder={n} -> {audio_s:.2f} s clip ({spec['baseline']})", "parallelism": f"host CPU, {cores} threads"},
         "cpu_baseline": base, "e2e": {"value": round(value, 5), "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     })
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(audio=g["audio"], semantic_tokens=g["semantic"], coarse_tokens=g["coarse"], fine_tokens=g["fine"]))
+
+
+def dump_outputs(out_dir, arrays):
+    """What the timed path returned in its last step, as out_dir/<name>.npy in float32 (token ids < 2^24 are exact), so that two
+    builds run with the same arguments (same seeded weights, prompt and seed) can be compared output for output.  Every
+    array is the whole output: a waveform of a clip and its token ids stay far below 64 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, np.float32))
 
 
 _REAL_STDOUT = None
@@ -608,6 +629,8 @@ def main():
     ap.add_argument("--no-fast", action="store_true", help="skip the extra fast-mode (tensor-core fine passes) leg")
     ap.add_argument("--cpu-budget", type=float, default=30.0)
     ap.add_argument("--config", default=None, choices=sorted(BENCH_CONFIGS), help="which BASELINE config to measure (default: bark-small f16 = configs[1])")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the waveform and token ids of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
     global BENCH_CONFIG
     if args.config:

@@ -31,3 +31,21 @@ def test_reference_arm_other_ranks_exit_quietly():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "0"],
                        capture_output=True, text=True, env=env, timeout=120)
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_dump_outputs_are_reproducible(tmp_path):
+    """--dump-outputs writes the last timed step's waveform and token ids as float32 .npy files; the same arguments give the
+    same inputs, so two runs write the same arrays."""
+    import numpy as np
+    env = dict(os.environ, BARK_B200_BENCH_CONFIG="tiny", BARK_B200_QUIET="1")
+    dumps = []
+    for run in ("a", "b"):
+        d = tmp_path / run
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "1", "--steps", "1", "--warmup", "0",
+                            "--dump-outputs", str(d)], capture_output=True, text=True, env=env, timeout=600)
+        assert r.returncode == 0, r.stderr[-800:]
+        dumps.append({p.stem: np.load(p) for p in sorted(d.glob("*.npy"))})
+    assert sorted(dumps[0]) == ["audio", "coarse_tokens", "fine_tokens", "semantic_tokens"]
+    for name, a in dumps[0].items():
+        assert a.dtype == np.float32 and a.size > 0, name
+        assert np.array_equal(a, dumps[1][name]), name

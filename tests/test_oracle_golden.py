@@ -15,8 +15,9 @@ def sha(a):
     return hashlib.sha1(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
-# small_* / large_*: true-size fixtures (tests/test_baseline_config0.py, tests/test_true_size_gpu.py); minutes of CPU time each on the oracle
-GOLDENS = sorted(p for p in glob.glob(os.path.join(GOLDEN_DIR, "*.npz")) if "gelu" not in p and not os.path.basename(p).startswith(("small_", "large_")))
+# small_* / large_*: true-size fixtures (tests/test_baseline_config0.py, tests/test_true_size_gpu.py); minutes of CPU time each on the oracle.
+# ref_checks.npz: the reference's answers for the inputs of other tests (tests/golden/make_golden_ref_checks.py)
+GOLDENS = sorted(p for p in glob.glob(os.path.join(GOLDEN_DIR, "*.npz")) if "gelu" not in p and not os.path.basename(p).startswith(("small_", "large_", "ref_checks")))
 
 
 def test_goldens_present():

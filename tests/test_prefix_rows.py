@@ -1,19 +1,16 @@
 """Canonical rows (bark_api.cu run_coarse, "Prefix reuse"): row p of a causal evaluation does not depend on the call's n_kv as
 long as p < n_kv & ~31, so a coarse window may start from the cached rows of the previous window.  Checked here on the CPU
-against the UNMODIFIED reference (oracle/_ref, where it travelled) and the C restatement: evaluating the tail of a sequence on
-top of the cached canonical rows gives bit-identical logits to evaluating the whole sequence from n_past = 0 — and a
-non-canonical row (p >= n_kv & ~31 of the call that produced it) does not."""
+on the C restatement, whose from-scratch logits must equal the UNMODIFIED reference's (tests/golden/ref_checks.npz, where the
+reference passed the same tail checks): evaluating the tail of a sequence on top of the cached canonical rows gives
+bit-identical logits to evaluating the whole sequence from n_past = 0 — and a non-canonical row (p >= n_kv & ~31 of the call
+that produced it) does not."""
+import hashlib
+import os
+
 import numpy as np
 import pytest
 
-from conftest import bits
-
-
-def engines(orc, path):
-    out = [("oracle", orc.Oracle(path))]
-    if orc.have_ref():
-        out.append(("reference", orc.Ref(path)))
-    return out
+from conftest import GOLDEN_DIR, bits
 
 
 @pytest.mark.parametrize("ftype", ["f32", "f16"])
@@ -21,20 +18,18 @@ def test_tail_on_canonical_rows_equals_from_scratch(orc, weights_file, ftype):
     path = weights_file("mini", ftype)
     rng = np.random.default_rng(21)
     full = np.concatenate([rng.integers(0, 10000, 256), [12050], rng.integers(10000, 12048, 75)]).astype(np.int32)
-    results = {}
-    for name, e in engines(orc, path):
-        scratch, p = e.gpt_eval(1, full, 0, False)
+    e = orc.Oracle(path)
+    scratch, p = e.gpt_eval(1, full, 0, False)
+    assert p == full.size
+    for cut in (256, 288, 320):
+        _, p = e.gpt_eval(1, full[:cut + 5], 0, False)          # rows [0, cut) canonical ((cut + 5) & ~31 == cut)
+        tail, p = e.gpt_eval(1, full[cut:], cut, False)
         assert p == full.size
-        for cut in (256, 288, 320):
-            _, p = e.gpt_eval(1, full[:cut + 5], 0, False)          # rows [0, cut) canonical ((cut + 5) & ~31 == cut)
-            tail, p = e.gpt_eval(1, full[cut:], cut, False)
-            assert p == full.size
-            assert np.array_equal(bits(tail), bits(scratch)), f"{name}: tail after {cut} cached rows: {int((tail != scratch).sum())} logits differ"
-        # the decode path of the same thing: one id on top of a cache whose last rows came from single-token steps is how the
-        # reference's own windows end; starting the NEXT window from those rows would not be exact
-        results[name] = scratch
-    if len(results) == 2:
-        assert np.array_equal(bits(results["oracle"]), bits(results["reference"]))
+        assert np.array_equal(bits(tail), bits(scratch)), f"oracle: tail after {cut} cached rows: {int((tail != scratch).sum())} logits differ"
+    # the decode path of the same thing: one id on top of a cache whose last rows came from single-token steps is how the
+    # reference's own windows end; starting the NEXT window from those rows would not be exact
+    want = str(np.load(os.path.join(GOLDEN_DIR, "ref_checks.npz"))[f"prefix_rows_{ftype}_sha1"])
+    assert hashlib.sha1(bits(scratch).tobytes()).hexdigest() == want, "from-scratch logits differ from the reference's"
 
 
 def test_rows_written_by_decode_steps_are_not_canonical(orc, weights_file):
