@@ -51,6 +51,7 @@ EXPORTS = [
     "bark_b200_profile_enable", "bark_b200_profile_report", "bark_b200_io_counters", "bark_b200_decode_timing", "bark_b200_decode_adapt",
     "bark_b200_shard_init", "bark_b200_shard_connect", "bark_b200_shard_nvlink_bytes",
     "bark_b200_fast_mode", "bark_b200_fast_gemm", "bark_b200_fast_attention",
+    "bark_b200_generate_audio_batch", "bark_b200_batch_audio", "bark_b200_batch_tokens", "bark_b200_batch_eval", "bark_b200_batch_stats",
     "ggml_time_init", "ggml_time_us", "ggml_time_ms", "ggml_init", "ggml_free",
 ]
 
@@ -128,6 +129,16 @@ def lib() -> C.CDLL:
     L.bark_b200_fast_gemm.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int]
     L.bark_b200_fast_attention.restype = C.c_int
     L.bark_b200_fast_attention.argtypes = [vp, vp, vp, vp, C.c_int, C.c_int, C.c_int]
+    L.bark_b200_generate_audio_batch.restype = C.c_bool
+    L.bark_b200_generate_audio_batch.argtypes = [vp, C.POINTER(C.c_char_p), C.POINTER(C.c_uint32), C.c_int]
+    L.bark_b200_batch_audio.restype = C.c_int
+    L.bark_b200_batch_audio.argtypes = [vp, C.c_int, f32p, C.c_int]
+    L.bark_b200_batch_tokens.restype = C.c_int
+    L.bark_b200_batch_tokens.argtypes = [vp, C.c_int, C.c_int, i32p, C.c_int]
+    L.bark_b200_batch_eval.restype = C.c_int
+    L.bark_b200_batch_eval.argtypes = [vp, C.c_int, C.c_int, i32p, C.c_int, i32p, C.c_int, f32p]
+    L.bark_b200_batch_stats.restype = C.c_int
+    L.bark_b200_batch_stats.argtypes = [vp, C.c_void_p]
     L.ggml_time_us.restype = C.c_int64
     _lib = L
     return L
@@ -286,6 +297,48 @@ class Bark:
 
     def layernorm_fallbacks(self) -> int:
         return int(lib().bark_b200_layernorm_fallbacks(self.ctx))
+
+    # ---- batched generation ----
+    def generate_batch(self, texts, seeds):
+        """Several prompts on this context's GPU in one call; item i equals a fresh context with seed seeds[i] generating texts[i].
+        Returns [(audio, [semantic, coarse, fine]), ...]; the context's own RNG and outputs are left as they were."""
+        n = len(texts)
+        if len(seeds) != n:
+            raise ValueError("one seed per prompt")
+        t = (C.c_char_p * n)(*[s.encode() for s in texts])
+        sd = (C.c_uint32 * n)(*seeds)
+        if not lib().bark_b200_generate_audio_batch(self.ctx, t, sd, n):
+            raise RuntimeError("bark_b200_generate_audio_batch failed (see stderr)")
+        out = []
+        for i in range(n):
+            m = lib().bark_b200_batch_audio(self.ctx, i, None, 0)
+            audio = np.zeros(m, np.float32)
+            lib().bark_b200_batch_audio(self.ctx, i, _p(audio), m)
+            toks = []
+            for stage in range(3):
+                k = lib().bark_b200_batch_tokens(self.ctx, i, stage, None, 0)
+                a = np.zeros(max(k, 1), np.int32)
+                lib().bark_b200_batch_tokens(self.ctx, i, stage, _p(a), k)
+                a = a[:k]
+                toks.append(a.reshape(-1, 2) if stage == 1 else a.reshape(-1, 8) if stage == 2 else a)
+            out.append((audio, toks))
+        return out
+
+    def batch_eval(self, which: int, prompts, next_ids) -> np.ndarray:
+        """Teacher-forced batched decode: prompts [n][len] into per-item caches, then next_ids [n][steps] as batched steps;
+        returns logits [n][steps][n_out_vocab]."""
+        p = np.ascontiguousarray(prompts, np.int32); x = np.ascontiguousarray(next_ids, np.int32)
+        n, ln = p.shape; steps = x.shape[1]
+        out = np.zeros((n, steps, int(self.hparams(which)[6])), np.float32)
+        if not lib().bark_b200_batch_eval(self.ctx, which, n, _p(p), ln, _p(x), steps, _p(out)):
+            raise RuntimeError("bark_b200_batch_eval failed")
+        return out
+
+    def batch_stats(self) -> dict:
+        """The last batch call: per-stage microseconds, batched decode steps, sampled rows replayed on the host."""
+        a = np.zeros(6, np.int64)
+        lib().bark_b200_batch_stats(self.ctx, _p(a))
+        return dict(zip(("semantic_us", "coarse_us", "fine_us", "codec_us", "batched_steps", "host_replays"), (int(v) for v in a)))
 
 
 def fast_gemm(A: np.ndarray, W: np.ndarray) -> np.ndarray:

@@ -17,6 +17,19 @@ struct ShardState {
     unsigned long long nvlink_bytes = 0;             // bytes this rank stored into peer memory (K / V rows, sampled ids)
 };
 
+// batched generation on the context's GPU (batch.cu): per-item KV caches, step scratch, and the results of the last batch call
+struct BatchItem { std::vector<int32_t> semantic, coarse, fine; std::vector<float> audio; };
+struct BatchState {
+    float * kv = nullptr; size_t slot_floats = 0; int slots = 0;   // one K + V cache region per item, sized for the larger causal model
+    float * qkv = nullptr, * logits = nullptr;                      // step scratch: [32][3E] QKV rows, [32][n_out] logit rows
+    double * h_u = nullptr, * d_u = nullptr;                        // sampling buffers of the batch (the single-prompt ones stay untouched)
+    int32_t * h_tok = nullptr, * d_tok = nullptr, * h_flags = nullptr, * d_flags = nullptr;
+    float * h_eos = nullptr, * d_eos = nullptr;
+    long long n_sample_calls = 0;
+    std::vector<BatchItem> items;                                   // results of the last successful bark_b200_generate_audio_batch
+    int64_t stats[6] = {0, 0, 0, 0, 0, 0};                          // its semantic / coarse / fine / codec microseconds, batched steps, host replays
+};
+
 struct bark_context {
     int device = 0;
     cudaStream_t stream = nullptr;
@@ -46,6 +59,7 @@ struct bark_context {
     __half * f_a16 = nullptr, * f_h16 = nullptr, * f_qk16 = nullptr, * f_vt16 = nullptr, * f_att16 = nullptr;   // [1024][E], [1024][4E], [1024][2E], [E][1024], [1024][E]
 
     ShardState shard;
+    BatchState batch;
 
     bark::Workspace ws;
     void * d_q8_sums = nullptr;                       // experimental q4_1 / q5_1: q8_1 block sums s = f16(d * sum(q))
@@ -88,7 +102,9 @@ void * ctx_alloc(bark_context * ctx, size_t bytes);
 
 // gpt_forward.cu — one evaluation of a causal model; mirrors bark_eval_encoder_internal (bark.cpp:1586-1643)
 // logits [lm_lo, lm_hi) are computed and copied to logits_host + lm_lo (lm_hi <= 0: all of them)
-bool gpt_eval(bark_context * ctx, GPTModel & m, const int32_t * tokens, int n, int * n_past, bool merge_ctx, float * logits_host, int lm_lo = 0, int lm_hi = 0);
+// kv_k / kv_v: the [L][block_size][E] K / V cache to work on (null: the model's own, mem_k / mem_v)
+bool gpt_eval(bark_context * ctx, GPTModel & m, const int32_t * tokens, int n, int * n_past, bool merge_ctx, float * logits_host, int lm_lo = 0, int lm_hi = 0,
+              float * kv_k = nullptr, float * kv_v = nullptr);
 void build_decode_tables(bark_context * ctx, GPTModel & m);
 // one non-causal pass of the fine model; mirrors bark_eval_fine_encoder_internal (bark.cpp:1907-1959)
 bool fine_eval(bark_context * ctx, const int32_t * in_buffer /*[8][1024]*/, int nn, float * logits_host /*[1024][n_out]*/);
@@ -106,8 +122,26 @@ struct FusedSample { int n; float temp; const double * d_u; int32_t * d_tok; int
 bool fused_sampler_available(const bark_context * ctx, const GPTModel & m, int samp_n);
 bool gpt_decode_chained(bark_context * ctx, GPTModel & m, const int32_t * d_token, int * n_past, int lm_lo, int lm_hi, const FusedSample * fs = nullptr);
 bool sample_device(bark_context * ctx, GPTModel & m, const float * d_logits, int ld, int n, int rows, float temp, int32_t * out_tok, float * out_eos);
+struct SampleBufs { double * h_u, * d_u; int32_t * h_tok, * d_tok, * h_flags, * d_flags; float * h_eos, * d_eos; };   // pinned host / device, one entry per row
+void sample_rows_sync(bark_context * ctx, const SampleBufs & b, const float * d_logits, int ld, int n, int rows, float temp, int tok_add, int force,
+                      int32_t * out_tok, float * out_eos, long long * replays);
 int32_t sample_token_given_u(const float * logits, int n, float temp, double u, float * eos_p);
 
 int64_t now_us();
+
+// bark_api.cu — stage pieces shared by the single-prompt stage loops and the batched ones (batch.cu)
+void tokenize_input(bark_context * ctx, const std::string & text);                  // -> ctx->tokens (513 ids)
+bool semantic_stop(const bark_context_params & P, int32_t tok, float eos_p);        // the semantic loop's stop test (bark.cpp:1675-1677)
+struct CoarsePlan { float stc_ratio; int max_semantic_history, n_steps, n_windows; };
+bool coarse_plan(const bark_context_params & P, size_t n_semantic, CoarsePlan * cp);     // false (with a message) when there is nothing to generate
+// ids to evaluate for the coarse window that starts after the samples in `out`, with prefix reuse against the cache content kv_ids /
+// kv_canon (updated for the window); *n_past = cached rows the evaluation starts from
+std::vector<int32_t> coarse_window_input(const bark_context_params & P, const CoarsePlan & cp, const std::vector<int32_t> & sem, const std::vector<int32_t> & out,
+                                         bool kv_reuse, std::vector<int32_t> & kv_ids, size_t & kv_canon, int * n_past);
+int  coarse_lo(const bark_context_params & P, int step);                            // offset of coarse step `step`'s codebook window in the vocabulary
+void coarse_codes(const bark_context_params & P, const std::vector<int32_t> & out, std::vector<int32_t> & codes);   // samples -> [T][2] codes
+bool run_fine(bark_context * ctx);                                                  // ctx->coarse_tokens -> ctx->fine_tokens, drawing from ctx->rng
+bool audio_params_supported(const bark_context_params & P);
+bool fine_to_audio(bark_context * ctx);                                             // ctx->fine_tokens -> ctx->audio (EnCodec)
 
 }  // namespace bark

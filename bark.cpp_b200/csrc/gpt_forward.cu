@@ -20,8 +20,9 @@ int64_t now_us() {
 
 // transformer body shared by the causal and the fine model; x [N][E] is updated in place.
 // K/V rows of this call go to k_dst/v_dst (KV-cache slot of position n_past, or the fine model's scratch),
-// attention then reads n_kv rows starting at k_all/v_all.
-static void run_layers(bark_context * ctx, GPTModel & m, int N, int n_past, bool causal) {
+// attention then reads n_kv rows starting at k_all/v_all.  Causal models: mem_k / mem_v is the [L][block_size][E] cache
+// the call works on (the model's own, or one item's of a batch, batch.cu).
+static void run_layers(bark_context * ctx, GPTModel & m, int N, int n_past, bool causal, float * mem_k = nullptr, float * mem_v = nullptr) {
     Workspace & ws = ctx->ws;
     cudaStream_t s = ctx->stream;
     const int E = m.n_embd, H = m.n_head;
@@ -35,7 +36,7 @@ static void run_layers(bark_context * ctx, GPTModel & m, int N, int n_past, bool
         layernorm_act(ws.x, N, E, L.ln_1_g, L.ln_1_b, ws.act, (WType) awt, kpE, ctx->d_ln_fallbacks, s);
         float * k_all, * v_all, * k_dst, * v_dst; int n_kv;
         if (causal) {
-            k_all = m.mem_k + (size_t) il * m.block_size * E; v_all = m.mem_v + (size_t) il * m.block_size * E;
+            k_all = mem_k + (size_t) il * m.block_size * E; v_all = mem_v + (size_t) il * m.block_size * E;
             k_dst = k_all + (size_t) n_past * E; v_dst = v_all + (size_t) n_past * E; n_kv = n_past + N;      // bark.cpp:1294-1300
         } else {
             k_all = k_dst = ws.kbuf; v_all = v_dst = ws.vbuf; n_kv = N;
@@ -139,7 +140,8 @@ static void decode_step(bark_context * ctx, GPTModel & m, int token, const int32
     ctx->tag_base += (unsigned) decode_tags_per_step(m.n_layer);
 }
 
-bool gpt_eval(bark_context * ctx, GPTModel & m, const int32_t * tokens, int n, int * n_past, bool merge_ctx, float * logits_host, int lm_lo, int lm_hi) {
+bool gpt_eval(bark_context * ctx, GPTModel & m, const int32_t * tokens, int n, int * n_past, bool merge_ctx, float * logits_host, int lm_lo, int lm_hi,
+              float * kv_k, float * kv_v) {
     if (!n_past) { fprintf(stderr, "%s: n_past is null\n", __func__); return false; }
     const int64_t t0 = now_us();
     Workspace & ws = ctx->ws;
@@ -152,8 +154,10 @@ bool gpt_eval(bark_context * ctx, GPTModel & m, const int32_t * tokens, int n, i
     for (int i = 0; i < n; i++) if (tokens[i] < 0 || tokens[i] >= m.n_in_vocab) {      // the embedding gather is unchecked on the device
         fprintf(stderr, "%s: token id %d at position %d is outside the model's input vocabulary (%d)\n", __func__, tokens[i], i, m.n_in_vocab); return false;
     }
+    const bool own_cache = !kv_k;                            // the persistent decode kernel works on the model's own cache only
+    if (own_cache) { kv_k = m.mem_k; kv_v = m.mem_v; }
     if (*n_past > 0 && N == 1) {
-        if (ctx->use_decode_kernel && m.decode_ok && *n_past + 1 <= m.block_size) {
+        if (own_cache && ctx->use_decode_kernel && m.decode_ok && *n_past + 1 <= m.block_size) {
             decode_step(ctx, m, tokens[0], nullptr, *n_past, lm_lo, lm_hi);
             ctx->last_logits = m.glogits;
             if (logits_host) {
@@ -174,7 +178,7 @@ bool gpt_eval(bark_context * ctx, GPTModel & m, const int32_t * tokens, int n, i
     memcpy(ctx->h_tok, tokens, (size_t) n * sizeof(int32_t));
     BARK_CUDA_CHECK(cudaMemcpyAsync(ws.tok, ctx->h_tok, (size_t) n * sizeof(int32_t), cudaMemcpyHostToDevice, s)); g_h2d_bytes += (size_t) n * sizeof(int32_t);
     gpt_embed_causal(m, ws.tok, N, *n_past, merge, ws.x, s);
-    run_layers(ctx, m, N, *n_past, true);
+    run_layers(ctx, m, N, *n_past, true, kv_k, kv_v);
     // final norm + lm_head on the last position only (bark.cpp:1391-1405)
     const int kpE = is_quant(m.wtype) ? E : ws.max_rows * kGmGroup;
     layernorm_act(ws.x + (size_t)(N - 1) * E, 1, E, m.ln_f_g, m.ln_f_b, ws.act, is_quant(m.wtype) ? W_Q4_0 : m.wtype, kpE, ctx->d_ln_fallbacks, s);
@@ -285,32 +289,37 @@ bool fine_eval_fast(bark_context * ctx, const int32_t * in_buffer, int nn, float
 // probability of the last logit) in out_tok / out_eos.  The RNG stream advances exactly as gpt_sample would advance it.
 bool sample_device(bark_context * ctx, GPTModel & m, const float * d_logits, int ld, int n, int rows, float temp, int32_t * out_tok, float * out_eos) {
     const int64_t t0 = now_us();
-    cudaStream_t s = ctx->stream;
     if (rows < 1 || rows > 1024 || n < 2 || (size_t) n * 4 > 64 * 1024) { fprintf(stderr, "%s: unsupported shape (%d rows of %d)\n", __func__, rows, n); return false; }
-    if (temp != 0.0f) {
-        for (int r = 0; r < rows; r++) ctx->h_u[r] = std::generate_canonical<double, 53>(ctx->rng);   // what discrete_distribution::operator() draws
-        BARK_CUDA_CHECK(cudaMemcpyAsync(ctx->d_u, ctx->h_u, (size_t) rows * sizeof(double), cudaMemcpyHostToDevice, s)); g_h2d_bytes += (size_t) rows * sizeof(double);
-    }
+    if (temp != 0.0f) for (int r = 0; r < rows; r++) ctx->h_u[r] = std::generate_canonical<double, 53>(ctx->rng);   // what discrete_distribution::operator() draws
     const int force = ctx->debug_flag_every > 0 && (ctx->n_sample_calls++ % ctx->debug_flag_every) == 0;
-    sample_rows(d_logits, ld, n, rows, temp, ctx->d_u, ctx->d_stok, 0, nullptr, ctx->d_seos, ctx->d_sflags, force, s);
-    BARK_CUDA_CHECK(cudaMemcpyAsync(ctx->h_stok, ctx->d_stok, (size_t) rows * 4, cudaMemcpyDeviceToHost, s));
-    BARK_CUDA_CHECK(cudaMemcpyAsync(ctx->h_sflags, ctx->d_sflags, (size_t) rows * 4, cudaMemcpyDeviceToHost, s));
-    BARK_CUDA_CHECK(cudaMemcpyAsync(ctx->h_seos, ctx->d_seos, (size_t) rows * 4, cudaMemcpyDeviceToHost, s)); g_d2h_bytes += (size_t) rows * 12;
-    BARK_CUDA_CHECK(cudaStreamSynchronize(s));
-    std::vector<float> row;
-    for (int r = 0; r < rows; r++) {
-        if (ctx->h_sflags[r]) {
-            row.resize((size_t) n);
-            BARK_CUDA_CHECK(cudaMemcpy(row.data(), d_logits + (size_t) r * ld, (size_t) n * 4, cudaMemcpyDeviceToHost)); g_d2h_bytes += (size_t) n * 4;
-            ctx->h_stok[r] = sample_token_given_u(row.data(), n, temp, ctx->h_u[r], &ctx->h_seos[r]);
-            ctx->n_sample_host_replays++;
-        }
-        out_tok[r] = ctx->h_stok[r];
-        if (out_eos) out_eos[r] = ctx->h_seos[r];
-    }
+    const SampleBufs b{ctx->h_u, ctx->d_u, ctx->h_stok, ctx->d_stok, ctx->h_sflags, ctx->d_sflags, ctx->h_seos, ctx->d_seos};
+    sample_rows_sync(ctx, b, d_logits, ld, n, rows, temp, 0, force, out_tok, out_eos, &ctx->n_sample_host_replays);
     m.t_sample_us += now_us() - t0;
     m.n_sample += rows;
     return true;
+}
+
+// sample_rows over `rows` rows whose uniforms are already in b.h_u, then one synchronisation and the host replay of flagged rows
+void sample_rows_sync(bark_context * ctx, const SampleBufs & b, const float * d_logits, int ld, int n, int rows, float temp, int tok_add, int force,
+                      int32_t * out_tok, float * out_eos, long long * replays) {
+    cudaStream_t s = ctx->stream;
+    if (temp != 0.0f) { BARK_CUDA_CHECK(cudaMemcpyAsync(b.d_u, b.h_u, (size_t) rows * sizeof(double), cudaMemcpyHostToDevice, s)); g_h2d_bytes += (size_t) rows * sizeof(double); }
+    sample_rows(d_logits, ld, n, rows, temp, b.d_u, b.d_tok, 0, nullptr, b.d_eos, b.d_flags, force, s);
+    BARK_CUDA_CHECK(cudaMemcpyAsync(b.h_tok, b.d_tok, (size_t) rows * 4, cudaMemcpyDeviceToHost, s));
+    BARK_CUDA_CHECK(cudaMemcpyAsync(b.h_flags, b.d_flags, (size_t) rows * 4, cudaMemcpyDeviceToHost, s));
+    BARK_CUDA_CHECK(cudaMemcpyAsync(b.h_eos, b.d_eos, (size_t) rows * 4, cudaMemcpyDeviceToHost, s)); g_d2h_bytes += (size_t) rows * 12;
+    BARK_CUDA_CHECK(cudaStreamSynchronize(s));
+    std::vector<float> row;
+    for (int r = 0; r < rows; r++) {
+        if (b.h_flags[r]) {
+            row.resize((size_t) n);
+            BARK_CUDA_CHECK(cudaMemcpy(row.data(), d_logits + (size_t) r * ld, (size_t) n * 4, cudaMemcpyDeviceToHost)); g_d2h_bytes += (size_t) n * 4;
+            b.h_tok[r] = sample_token_given_u(row.data(), n, temp, b.h_u[r], &b.h_eos[r]);
+            ++*replays;
+        }
+        out_tok[r] = tok_add + b.h_tok[r];
+        if (out_eos) out_eos[r] = b.h_eos[r];
+    }
 }
 
 bool codec_decode(bark_context * ctx, const int32_t * codes, int T) {

@@ -64,6 +64,18 @@ bool fast_gemm(const __half * A, int lda, const __half * W, int ldw, int M, int 
 bool fast_attention(const __half * qk, int ldq, int k_col0, const __half * vt, int n, int E, int H, __half * out, cudaStream_t s);
 void fast_layernorm(const float * x, int rows, int E, const float * g, const float * b, __half * out, cudaStream_t s);
 
+// ---- batched decode step (batch_kernels.cu; driven by batch.cu): B <= kBatchMax items, one new position each, all at the same n_past ----
+constexpr int kBatchMax = 32;                        // one row tile (kBM) of lane_gemm_tiled_kernel: every mat-mul of a step is one row tile
+struct RowIds { int32_t v[kBatchMax]; };             // one input id per row, passed by value
+struct BatchKV { float * k[kBatchMax]; float * v[kBatchMax]; };   // per row: the item's K / V cache of the current layer, [block_size][E] f32
+// x[b] = wte[tok[b]] + wpe[pos] for rows b < B (every weight type the loader accepts)
+void gpt_embed_rows(const GPTModel & m, const RowIds & tok, int B, int pos, float * x, cudaStream_t s);
+void qx_embed_rows(const GPTModel & m, const RowIds & tok, int B, int pos, float * x, cudaStream_t s);
+// one layer's attention for B decode rows: appends each row's K / V slice (qkv [B][3E]) to its cache at n_past, then scores, soft_max
+// and P.V over n_past + 1 keys in the reference's order; the result goes to the next mat-mul's operand (store_act)
+void batch_decode_attention(const float * qkv, const BatchKV & kv, int B, int n_past, int E, int H, void * act, WType wt, int Kp,
+                            unsigned * softmax_fallbacks, cudaStream_t s);
+
 // ---- persistent decode step (decode_kernels.cu) -----------------------------------------------------------------
 constexpr int kDecodeReplicas = 8;        // copies of each all-to-all exchange vector (gx, gq, gatt, gff): CTA c reads copy c % 8
 struct DecodePhase { const void * w; int n_out, row_bytes, K, pad; const void * ws; };   // one streamed matrix: LI rows (f32 / f16), or q4_0 nibble words (16 B per block) with f16 block scales in ws

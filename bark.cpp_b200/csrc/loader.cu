@@ -106,7 +106,7 @@ bool load_gpt(bark_context * ctx, std::ifstream & f, GPTModel & m, const char * 
     auto vec = [&](const std::string & n, float ** p, int len) { Slot s{Slot::VEC, len, 1}; s.vec = p; slots[n] = s; };
     auto mat = [&](const std::string & n, DMat * p, int K, int O, bool gm) { Slot s{Slot::MATRIX, K, O}; s.mat = p; s.gm = gm; slots[n] = s; };
     for (int i = 0; i < m.n_wtes; i++) { Slot s{Slot::TABLE, E, m.n_in_vocab}; s.table = &m.wte[i]; slots["model/wte/" + std::to_string(i)] = s; }
-    for (int i = 0; i < m.n_lm_heads; i++) mat("model/lm_head/" + std::to_string(i), &m.lm_head[i], E, m.n_out_vocab, !causal);   // causal models apply lm_head to one row only
+    for (int i = 0; i < m.n_lm_heads; i++) mat("model/lm_head/" + std::to_string(i), &m.lm_head[i], E, m.n_out_vocab, true);   // causal models: one row, or the 16-32 rows of a batched step (batch.cu)
     { Slot s{Slot::WPE, E, m.block_size}; s.vec = &m.wpe; slots["model/wpe"] = s; }
     vec("model/ln_f/g", &m.ln_f_g, E);
     if (m.bias) vec("model/ln_f/b", &m.ln_f_b, E);

@@ -44,6 +44,10 @@ __global__ void embed_causal_q_kernel(const void * __restrict__ wte, int wt, con
         x[(size_t) r * E + i] = __fadd_rn(v, wpe[(size_t)(r + n_past) * E + i]);
     }
 }
+__global__ void embed_rows_q_kernel(const void * __restrict__ wte, int wt, const float * __restrict__ wpe, RowIds tok, int pos, int E, float * __restrict__ x) {
+    const int r = blockIdx.x;
+    for (int i = threadIdx.x; i < E; i += blockDim.x) x[(size_t) r * E + i] = __fadd_rn(wte_value_q(wte, wt, E, tok.v[r], i), wpe[(size_t) pos * E + i]);
+}
 struct FineTablesQ { const void * wte[8]; };
 __global__ void embed_fine_q_kernel(FineTablesQ tabs, int wt, const float * __restrict__ wpe, const int32_t * __restrict__ ids, int nn, int E, float * __restrict__ x) {
     const int r = blockIdx.x;
@@ -161,6 +165,9 @@ void qx_set_scratch(void * q8, void * q8_scales, void * q8_sums) { g_qx_q8 = (in
 
 void qx_embed_causal(const GPTModel & m, const int32_t * d_tok, int N, int n_past, bool merge, float * x, cudaStream_t s) {
     BARK_LAUNCH(embed_causal_q_kernel, N, 256, 0, s, m.wte[0], (int) m.wtype, m.wpe, d_tok, N, n_past, merge ? 1 : 0, m.n_embd, x);
+}
+void qx_embed_rows(const GPTModel & m, const RowIds & tok, int B, int pos, float * x, cudaStream_t s) {
+    BARK_LAUNCH(embed_rows_q_kernel, B, 256, 0, s, m.wte[0], (int) m.wtype, m.wpe, tok, pos, m.n_embd, x);
 }
 void qx_embed_fine(const GPTModel & m, const int32_t * d_ids, int nn, float * x, cudaStream_t s) {
     FineTablesQ t; for (int i = 0; i < 8; i++) t.wte[i] = m.wte[i];

@@ -80,6 +80,22 @@ BARK_API int  bark_b200_fast_mode(struct bark_context * ctx);              /* 1 
 BARK_API int  bark_b200_fast_gemm(const uint16_t * A, const uint16_t * W, float * C, int M, int N, int K);
 BARK_API int  bark_b200_fast_attention(const uint16_t * q, const uint16_t * k, const uint16_t * v, uint16_t * out, int n, int E, int H);
 
+/* BATCHED GENERATION on the context's GPU (csrc/batch.cu).  Item i's semantic / coarse / fine ids and waveform are bit-identical to
+ * bark_load_model(same file, same params, seeds[i]) followed by ONE bark_generate_audio(texts[i]).  1 <= n <= 32.  The semantic and coarse
+ * decode steps of all items run as one batched step; the fine and EnCodec stages run item by item.  The call leaves the context's
+ * single-prompt state alone (RNG, token arrays, bark_get_audio_data, statistics) and reports no progress.  Returns false (message on
+ * stderr) on bad arguments, a sharded context, unsupported audio parameters or too little device memory. */
+BARK_API bool bark_b200_generate_audio_batch(struct bark_context * ctx, const char * const * texts, const uint32_t * seeds, int n);
+BARK_API int  bark_b200_batch_audio(struct bark_context * ctx, int item, float * out, int cap);                 /* sample count, copies min(count, cap); -1 on a bad item */
+BARK_API int  bark_b200_batch_tokens(struct bark_context * ctx, int item, int stage, int32_t * out, int cap);  /* stage as bark_b200_get_tokens (0, 1, 2) */
+/* test hook: teacher-forced batched decode.  which: 0 semantic, 1 coarse.  Every item's `len` prompt ids are evaluated into the
+ * item's own KV cache (n_past 0, no merge), then `steps` batched single-token steps with next[i][j]; logits_out [n][steps][n_out_vocab].
+ * Returns 1, or 0 on failure. */
+BARK_API int  bark_b200_batch_eval(struct bark_context * ctx, int which, int n, const int32_t * prompts /*[n][len]*/, int len,
+                                   const int32_t * next /*[n][steps]*/, int steps, float * logits_out);
+/* the last batch call: {semantic, coarse, fine, EnCodec} microseconds, batched decode steps, sampled rows replayed on the host */
+BARK_API int  bark_b200_batch_stats(struct bark_context * ctx, int64_t * out6);
+
 #ifdef __cplusplus
 }
 #endif
